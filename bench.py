@@ -4,6 +4,7 @@
 Contract (see DESIGN.md §Measurement):
   python bench.py --gpus N --steps K --warmup W            # our arm (torchrun for N > 1, one rank per GPU)
   python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU path (oracle port) on host cores
+  python bench.py ... --dump-outputs DIR                   # also write the last timed step's outputs as DIR/<name>.npy
 
 One bench "step" = one complete sample of the batch: T reverse-diffusion steps + the final decode
 (T+1 denoiser forwards), i.e. BASELINE.json's metric "molecules/sec (1000-step sample)".  Workload at N=1 is
@@ -51,7 +52,34 @@ def parse_args():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--cpu-forwards", type=int, default=0,
                     help="denoiser forwards per CPU sample (bounded sample of the workload; default 8, geom_hist 2)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step returned as DIR/<name>.npy (float32)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
+    return args
+
+
+DUMP_MAX_BYTES = 64 * 1000 * 1000
+
+
+def dump_outputs(dirname, arrays):
+    """Write each tensor of `arrays` (name -> tensor) as `dirname`/<name>.npy in float32.  Past 64 MB in all, every array
+    is flattened and cut to the same fraction of its elements (at least one), taken at seeded (hence fixed) positions, so
+    that two builds run with the same arguments can still be compared element for element."""
+    import numpy as np
+    os.makedirs(dirname, exist_ok=True)
+    host = {k: v.detach().to("cpu", torch.float32) for k, v in arrays.items()}
+    total = sum(4 * v.numel() for v in host.values())
+    budget = DUMP_MAX_BYTES - (128 + 4) * len(host)                  # per file: .npy header, the one element always kept
+    for name, v in host.items():
+        keep = max(1, v.numel() * budget // max(total, 1))
+        if keep < v.numel():
+            idx = torch.randperm(v.numel(), generator=torch.Generator().manual_seed(0))[:keep].sort().values
+            v = v.reshape(-1)[idx]
+        np.save(os.path.join(dirname, name + ".npy"), v.numpy())
 
 
 # ------------------------------------------------------------------------------------------------ clocks
@@ -177,7 +205,7 @@ def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    block, secs, desc = cpu_arm(args, reps=max(1, min(args.steps, 3)))
+    block, secs, desc = cpu_arm(args, reps=args.steps)
     line = {
         "impl": "reference", "metric": METRIC, "value": block["value"], "unit": "molecules/s", "n_gpus": args.gpus,
         "steps": args.steps, "warmup": args.warmup, "ms_per_step": 1000 * secs, "higher_is_better": True,
@@ -239,17 +267,21 @@ def run_ours(args):
     out_host = torch.empty((int(sizes_all.sum()) if strong else n_nodes, width), pin_memory=True)
     flush_buf = torch.empty(256 * 1024 * 1024 // 4, device=dev)      # > 126 MB L2
     finite_flag = torch.ones((), dtype=torch.bool, device=dev)
+    last = []                                                        # the job's samples from the latest chain
 
     def one_chain(nodes, ctx):
         """The product's public call for this workload; returns the step's result on the device."""
         nonlocal finite_flag
         if strong:
             out, _ = sample_sharded(sampler, nodes, ctx, T)          # LPT shards, chain, ONE NCCL all_gather
+            last[:] = [out]
         else:
             out, _, _ = sampler.sample(nodes, ctx, T)
+            last[:] = [out]
             if world > 1:
                 bufs = [torch.empty_like(out) for _ in range(world)]
                 dist.all_gather(bufs, out)                           # single NCCL gather of final coordinates
+                last[:] = bufs
         finite_flag = finite_flag & torch.isfinite(out).all()
         return out
 
@@ -304,6 +336,7 @@ def run_ours(args):
     if rank == 0:
         clocks.start()
     secs = timed(chain_resident, args.steps)
+    final = list(last)                                               # outputs of the last timed chain
     clk = clocks.stop() if rank == 0 else None
     launches = sampler_launches(sampler, net) - launches0
     log(f"timed resident chains done: {secs:.2f} s for {args.steps}")
@@ -482,6 +515,8 @@ def run_ours(args):
         line["gpu_unfused_baseline"] = gpu_unfused
     if world == 1 and rank == 0 and not args.no_cpu_baseline:
         line["cpu_baseline"] = cpu_arm(args, reps=1)[0]
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"samples": torch.cat(final)})     # [molecules x atoms, 3 + atom types (+1)]
     if rank == 0:
         print(json.dumps(line), flush=True)
     if world > 1:
@@ -519,6 +554,7 @@ def run_train(args):
     net.set_train_precision(args.train_tf32)
     opt = GCDMTrainTail(net.parameters())
     tl = bdiff.GCDMTrainLoss(net, GEOM_N_NODES)
+    torch.manual_seed(123 + rank)                                # t and the noise of every step: same in every run
     B = args.batch or 64
     nb = 4                                                       # distinct host batches, cycled
     A = dcfg.num_atom_types
@@ -538,6 +574,7 @@ def run_train(args):
     flush_buf = torch.empty(256 * 1024 * 1024 // 4, device=dev)
     counter = [0]
     finite = [True]
+    last = [None]                                                # loss of the latest resident step
 
     def train_step(batch):
         opt.zero_grad()
@@ -550,6 +587,7 @@ def run_train(args):
     def step_resident():
         loss = train_step(dev_batches[counter[0] % nb])
         counter[0] += 1
+        last[0] = loss
         return loss
 
     def step_e2e():
@@ -595,6 +633,9 @@ def run_train(args):
     secs = timed(step_resident, args.steps)
     clk = clocks.stop() if rank == 0 else None
     launches = (net.launch_count() - l0) + (opt.kernel_launches - k0)
+    final = None
+    if args.dump_outputs:                                        # the last timed step's loss and the weights it left
+        final = {"loss": last[0], "parameters": torch.cat([p.detach().reshape(-1) for p in net.parameters()])}
     counter[0] = 0
     secs_e2e = timed(step_e2e, args.steps)
     fin = torch.tensor([int(finite[0])], device=dev)
@@ -671,6 +712,8 @@ def run_train(args):
         line["cpu_baseline"] = {"value": cpu_mols / dt, "unit": "molecules/s", "cores": torch.get_num_threads(), "kind": "port",
                                 "sample": f"one forward+backward (torch autograd through the oracle port) of the first {cpu_mols} "
                                           f"molecules of batch 0 ({nn0} atoms), {dt:.1f} s"}
+    if rank == 0 and final is not None:
+        dump_outputs(args.dump_outputs, final)
     if rank == 0:
         print(json.dumps(line), flush=True)
     if world > 1:

@@ -18,9 +18,11 @@ ref_shim.install()      # stub modules + /root/reference on sys.path
 from src.models import Queue, get_grad_norm  # noqa: E402
 
 torch.manual_seed(11)
+# the inputs (initial parameters, gradients) are drawn on the float16 grid and stored as float16, which is exact and keeps
+# the fixture small; the last tensor spans two chunks of the optimiser kernels (bdiff_optimizer_chunk = 16384)
 shapes = [(64, 77), (64,), (32, 8), (1, 64), (17,), (20000,)]
-params = [torch.nn.Parameter(torch.randn(s) * 0.1) for s in shapes]
-init = [p.detach().clone() for p in params]
+init = [(torch.randn(s) * 0.1).half() for s in shapes]
+params = [torch.nn.Parameter(p.float()) for p in init]
 opt = torch.optim.AdamW(params, lr=1e-4, weight_decay=1e-12, amsgrad=True)
 queue = Queue()
 queue.add(3000)
@@ -29,9 +31,9 @@ decay = 0.9999
 steps, log = [], []
 scales = [1.0, 0.5, 2.0, 4000.0, 1.0, 300.0, 1.0, 1.0]          # two spikes exercise the clipping branch
 for k, sc in enumerate(scales):
-    grads = [torch.randn(s) * sc for s in shapes]
+    grads = [(torch.randn(s) * sc).half() for s in shapes]
     for p, g in zip(params, grads):
-        p.grad = g.clone()
+        p.grad = g.float()
     limit = 1.5 * queue.mean() + 2 * queue.std()
     norm = get_grad_norm(params)
     torch.nn.utils.clip_grad_norm_(params, max_norm=float(limit), norm_type=2.0)

@@ -1,13 +1,11 @@
 """GPU: bdiff_optimizer_step (clipping + AdamW(amsgrad) + EMA in three multi-tensor kernels) against the oracle and the
 golden fixture produced with the reference's own pieces.  Tolerance: fp32 elementwise arithmetic, 2e-6 relative on
 parameters / EMA (the kernel contracts a*b+c into FMAs; torch does not), gradient norm 1e-6 relative."""
-import os
-
 import pytest
 import torch
 
 import optim_oracle as OO
-from conftest import GOLDEN
+from test_optim_oracle import load as load_fixture
 
 pytestmark = pytest.mark.gpu
 
@@ -15,7 +13,7 @@ pytestmark = pytest.mark.gpu
 def test_train_tail_matches_oracle_and_fixture():
     import bdiff
     from bdiff.optim import GCDMTrainTail
-    fx = torch.load(os.path.join(GOLDEN, "optim_steps.pt"), weights_only=False)
+    fx = load_fixture()
     params = [torch.nn.Parameter(p.clone().cuda()) for p in fx["init"]]
     opt = GCDMTrainTail(params)
     orc = OO.TrainTailOracle(fx["init"])

@@ -9,7 +9,11 @@ from conftest import GOLDEN
 
 
 def load():
-    return torch.load(os.path.join(GOLDEN, "optim_steps.pt"), weights_only=False)
+    """The fixture, its float16-stored inputs (exact: drawn on the float16 grid) widened to the float32 they are used in."""
+    fx = torch.load(os.path.join(GOLDEN, "optim_steps.pt"), weights_only=False)
+    fx["init"] = [p.float() for p in fx["init"]]
+    fx["grads"] = [[g.float() for g in step] for step in fx["grads"]]
+    return fx
 
 
 def test_oracle_matches_reference_pieces():
