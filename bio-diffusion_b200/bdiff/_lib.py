@@ -36,6 +36,7 @@ PROTOTYPES = {
     "bdiff_prepare": (C.c_int32, [C.c_void_p, C.c_void_p]),
     "bdiff_selftest_split": (C.c_int32, [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]),
     "bdiff_selftest_pair": (C.c_int32, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "bdiff_tc_edge_stream_layout": (C.c_int32, [C.c_int32, C.c_int32, C.POINTER(C.c_int64)]),
     "bdiff_plan_topology": (C.c_int32, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int64, C.c_void_p, C.c_void_p,
                                         C.POINTER(C.c_int64)]),
     "bdiff_edge_index": (C.c_int32, [C.c_void_p, C.c_void_p, C.c_void_p]),

@@ -202,6 +202,12 @@ extern "C" {
 
 int32_t bdiff_abi_version(void) { return BDIFF_ABI_VERSION; }
 
+int32_t bdiff_tc_edge_stream_layout(int32_t e_hidden, int32_t xi_hidden, int64_t* out) {
+  if (!out || !tc_supported(e_hidden, xi_hidden)) return BDIFF_EINVAL;
+  tc_edge_stream_layout(e_hidden, xi_hidden, out);
+  return 0;
+}
+
 const char* bdiff_last_error(const bdiff_handle* h) { return h ? h->err.c_str() : g_create_error.c_str(); }
 
 int32_t bdiff_create(const bdiff_config* cfg, bdiff_handle** out) {

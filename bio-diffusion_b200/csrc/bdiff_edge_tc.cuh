@@ -9,23 +9,48 @@ namespace bdiff {
 constexpr int TMT = 128;                 // edges per tile
 // weight ring: TC_NSLOT slots of TC_SLOT bytes; a chunk is one slab plane (N rows x 32 B, N <= 320) or a group of
 // small planes, always a single contiguous TMA bulk copy
-constexpr int TC_SLOT = 2 * 160 * 32;    // 10 KiB: this CTA's half of the widest K step (hi plane + lo plane)
+constexpr int TC_SLOT = 2 * 160 * 32;    // 10 KiB: holds the widest chunk (9 KiB: a node-tile K step of 144 local rows, hi + lo)
 constexpr int TC_NSLOT = 5;
 // TMEM column map of an edge tile (512 columns allocated)
 constexpr int TM_S = 0, TM_U0 = 256, TM_U1 = 288, TM_MV = 320, TM_VD0 = 416;
 constexpr int TM_EX = 416, TM_EX_STRIDE = 40;     // pair-exchange scratch (over VD0, which is dead by then): 2 x 40 columns
 
-__host__ __device__ inline int tc_k0_steps(int Ed, int Xd) {     // K=16 steps of message GCP 0's edge part
+__host__ __device__ constexpr int tc_k0_steps(int Ed, int Xd) {     // K=16 steps of message GCP 0's edge part
   return (Ed + (64 + Xd) / 4 + 9 + 15) / 16;
 }
 // bytes of one layer's edge-pass weight stream (see k_pack_edge_slabs for the order)
-__host__ __device__ inline size_t tc_edge_stream_bytes(int Ed, int Xd) {
+__host__ __device__ constexpr size_t tc_edge_stream_bytes(int Ed, int Xd) {
   return (size_t)tc_k0_steps(Ed, Xd) * 2 * 256 * 32 + 3 * ((size_t)16 * 2 * 320 * 32 + 2 * 2 * 256 * 32) + (size_t)16 * 2 * 32 * 32;
 }
 
-// mbarriers / bookkeeping of the megakernel; first member (base class) of both tile tails
+// One CTA's half of an edge tile's weight stream as TMA chunks (one bulk copy and one ring slot each), in issue order:
+//   G0                      k0s chunks: one K step of 128 rows ([hi plane | lo plane])
+//   k = 1..3   U pass         4 chunks: 4 K steps of the 32 gate rows each
+//              S pass        16 chunks: one K step of 128 rows of W_k
+//              G(k)b          2 chunks: one K step of 128 rows (W_k K rows 256..287)
+//   G4                        4 chunks: 4 K steps of 16 rows of Wg_3 each
+// The TMA producer streams exactly these chunks and the peer's relay lane forwards one completion per chunk, so both
+// take their count from here.
+constexpr uint32_t TC_EC_S = 2 * 128 * 32, TC_EC_U = 4 * 2 * 32 * 32, TC_EC_G4 = 4 * 2 * 16 * 32;
+constexpr int TC_EC_PER_GCP = 4 + 16 + 2;
+__host__ __device__ constexpr int tc_edge_tile_chunks(int k0s) { return k0s + 3 * TC_EC_PER_GCP + 4; }
+__host__ __device__ constexpr uint32_t tc_edge_chunk_bytes(int k0s, int c) {
+  return c < k0s ? TC_EC_S : c < k0s + 3 * TC_EC_PER_GCP ? ((c - k0s) % TC_EC_PER_GCP < 4 ? TC_EC_U : TC_EC_S) : TC_EC_G4;
+}
+__host__ __device__ constexpr size_t tc_edge_chunks_total_bytes(int k0s) {     // both CTAs
+  size_t b = 0;
+  for (int c = 0; c < tc_edge_tile_chunks(k0s); ++c) b += tc_edge_chunk_bytes(k0s, c);
+  return 2 * b;
+}
+static_assert(tc_edge_chunks_total_bytes(tc_k0_steps(64, 16)) == tc_edge_stream_bytes(64, 16) &&
+              tc_edge_chunks_total_bytes(tc_k0_steps(16, 8)) == tc_edge_stream_bytes(16, 8),
+              "edge chunk table and packed stream size disagree");
+static_assert(TC_EC_S <= TC_SLOT && TC_EC_U <= TC_SLOT && TC_EC_G4 <= TC_SLOT, "an edge chunk fits one ring slot");
+
+// mbarriers / bookkeeping of the megakernel; first member (base class) of both tile tails.  u_full: the gate pass of an
+// edge GCP is complete (its own commit, ahead of the S pass that d_full waits for).
 struct TcBars {
-  uint64_t full[TC_NSLOT], empty[TC_NSLOT], pfull[TC_NSLOT], a_ready, d_full, wbar, u_free;
+  uint64_t full[TC_NSLOT], empty[TC_NSLOT], pfull[TC_NSLOT], a_ready, d_full, wbar, u_free, u_full;
   uint64_t item_full[2], item_empty[2], peer_empty[2], tile_done;
   alignas(16) int item[2][4];   // work items {type, layer, tile of THIS CTA, -}; the leader writes the peer's copy (16-byte st.shared::cluster)
   uint32_t tmem_ptr;

@@ -62,6 +62,7 @@ void launch_pack_multi(cudaStream_t st, const PackJob* jobs_dev, int njobs, int 
 // tensor mode: per-layer split-bf16 weight streams (bdiff_tc_pack.cu)
 bool tc_supported(int Ed, int Xd);
 size_t tc_blob_bytes(int Ed, int Xd);
+void tc_edge_stream_layout(int Ed, int Xd, int64_t* out);   // {stream bytes, chunks per CTA and tile, chunk bytes of both CTAs}
 size_t tc_node_blob_bytes();
 void launch_tc_pack(cudaStream_t st, const LayerW& lw, const Dims& d, unsigned char* blob);
 void launch_tc_pack_node(cudaStream_t st, const LayerW& lw, const LayerW& wn, const EmbedW& ew, const Dims& d, int last,

@@ -111,6 +111,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(LAYERS_THREADS, 1)
     mbar_init(&B.tile_done, TC_EPI);
     mbar_init(&B.a_ready, leader ? TC_EPI + 1 : TC_EPI);   // leader's: its own compute threads + ONE arrival relayed by the peer's MMA lane
     mbar_init(&B.d_full, 1);
+    mbar_init(&B.u_full, 1);
     mbar_init(&B.wbar, 1);
     mbar_init(&B.u_free, leader ? TC_EPI + 1 : TC_EPI);
     mbar_fence_init();
@@ -189,7 +190,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(LAYERS_THREADS, 1)
         mbar_wait_cluster(&B.item_full[slot], (k >> 1) & 1);
         const int type = B.item[slot][0], layer = B.item[slot][1], tile = B.item[slot][2];
         if (type < 0) break;
-        const uint32_t nch = type == 0 ? K0S + 3 * 18 + 4 : (layer == q.L - 1 ? 73u : 100u);      // chunks per tile (producer includes)
+        const uint32_t nch = type == 0 ? (uint32_t)tc_edge_tile_chunks(K0S) : (layer == q.L - 1 ? 73u : 100u);   // chunks per tile (producer includes)
         // lane = ring slot: a lane sees the phases of ITS slot's barrier strictly in order (waiting for a phase two uses ahead
         // would alias with the parity of the current one)
         for (uint32_t cc = ci + ((lane + TC_NSLOT - ci % TC_NSLOT) % TC_NSLOT); cc < ci + nch; cc += TC_NSLOT) {
@@ -233,6 +234,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(LAYERS_THREADS, 1)
       };
       auto done_w = [&]() { if (leader) umma_commit_pair(&B.empty[ci % TC_NSLOT]); ++ci; };
       auto commit_d = [&]() { if (leader) umma_commit_pair(&B.d_full); };
+      auto commit_u = [&]() { if (leader) umma_commit_pair(&B.u_full); };
       auto mma = [&](uint32_t dcol, uint64_t ad, uint64_t bd, uint32_t idesc, bool acc) { if (leader) umma_bf16_pair(tmem + dcol, ad, bd, idesc, acc); };
       // node-tile GEMMs over A blocks 0..3 (R5 layout: views at row 0 and row 32, four products per K step).  Local plane =
       // [128 rows of the S columns | 16 gate rows] (NL rows): S is one N=256 pair MMA, the gate accumulator U (columns 256..287)
@@ -320,7 +322,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(LAYERS_THREADS, 1)
   } else {
     // ============================================================================ compute / epilogue warps
     asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;\n" ::"n"(LAYERS_REG_COMPUTE));
-    uint32_t pd = 0, pw = 0;
+    uint32_t pd = 0, pg = 0, pw = 0;
     int cur_type = -1, cur_layer = -1;
     // BDIFF_TIMING: phase stamps (clock64) of the first edge / node item with k >= 2 of every CTA: [128 + 0..31] edge,
     // [128 + 32..63] node — one stamp before and after every accumulator wait, one after every operand publication
@@ -328,6 +330,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(LAYERS_THREADS, 1)
     long long* stamp = nullptr;
     auto PH = [&]() { if (stamp && tid == 0 && es < 32) stamp[es] = clock64(); ++es; };
     auto wait_d = [&]() { PH(); mbar_wait(&B.d_full, pd); pd ^= 1; tc_fence_after(); PH(); };
+    auto wait_u = [&]() { PH(); mbar_wait(&B.u_full, pg); pg ^= 1; tc_fence_after(); PH(); };     // edge tiles: gate pass done
     auto publish = [&]() { fence_proxy_async(); tc_fence_before(); mbar_arrive(&B.a_ready); PH(); };
     bool stamped[2] = {false, false};
     const uint32_t tl = tmem + ((uint32_t)((warp & 3) * 32) << 16);

@@ -6,13 +6,21 @@ namespace bdiff {
 
 size_t tc_blob_bytes(int Ed, int Xd) { return tc_edge_stream_bytes(Ed, Xd); }
 size_t tc_node_blob_bytes() { return tc_node_stream_bytes(0); }      // the last layer's stream is shorter
+void tc_edge_stream_layout(int Ed, int Xd, int64_t* out) {
+  const int k0s = tc_k0_steps(Ed, Xd);
+  out[0] = (int64_t)tc_edge_stream_bytes(Ed, Xd);
+  out[1] = tc_edge_tile_chunks(k0s);
+  out[2] = (int64_t)tc_edge_chunks_total_bytes(k0s);
+}
 
 // A layer's stream is [CTA 0's half | CTA 1's half] (the megakernel runs CTA pairs, cta_group::2: an N-row plane is split between
 // the two shared memories, CTA c supplying rows [c N/2, (c+1) N/2) of every MMA's B operand).  Per CTA, in streaming order:
 // Edge pass:  G0: K0S steps x 128 local rows (W0e rows [128 c, 128 c + 128), zero-padded to K0S*16 K rows)
-//             for k = 1..3:  16 steps x 160 local rows = [W_k rows 128 c .. +128 | 32 gate rows: CTA 0 -> U0, CTA 1 -> U1],
+//             for k = 1..3:  U pass: 16 steps x 32 local gate rows (CTA 0 -> U0, CTA 1 -> U1), 4 steps per TMA chunk,
+//                            S pass: 16 steps x 128 local rows (W_k rows 128 c .. +128),
 //                            2 steps x 128 local rows (W_k K rows 256..287)
 //             G4: 16 steps x 16 local rows (Wg_3 rows [16 c, 16 c + 16))
+//             (tc_edge_chunk_bytes lists the TMA chunks of this order)
 // Gate rows: GCP kk = gi + 1 adds +Wg_{kk-1} m_{kk-1} to U[(kk-1) & 1] and starts U[kk & 1] = -Wg_kk m_{kk-1} (sign folded into
 // the packed weights so that U0 | U1 is one N=64 accumulator range).
 // one thread per (global plane row, k in [0,16)); writes the hi and the lo plane element
@@ -40,14 +48,21 @@ __global__ void k_pack_edge_slabs(LayerW lw, Dims d, unsigned char* __restrict__
       long long rr = row - gi * rows_g;
       base += gi * bytes_g;
       if (rr < 16 * 320) {
+        // global row n of K step `step`: W_k rows 0..255 go to the S pass (planes of 128 local rows, after the 16 gate
+        // planes), the 64 gate rows to the U pass (planes of 32 local rows, 4 K steps per chunk)
         const int step = (int)(rr / 320);
-        n = (int)(rr % 320); NL = 160; base += (size_t)step * 2 * 160 * 32; k = step * 16 + kk;
+        n = (int)(rr % 320); k = step * 16 + kk;
         const float* wprev = gi == 0 ? lw.Wg0 : lw.Wgk[gi - 1];
         const float* wthis = lw.Wgk[gi];
         const bool odd = ((gi + 1) & 1) != 0;           // kk odd: U0 <- +prev, U1 <- -this;  kk even: U0 <- -this, U1 <- +prev
-        if (n < 256) { v = lw.Wk[gi][(size_t)k * 256 + n]; cta = n >> 7; local = n & 127; }
-        else if (n < 288) { v = odd ? wprev[(size_t)k * 32 + (n - 256)] : -wthis[(size_t)k * 32 + (n - 256)]; cta = 0; local = 128 + (n - 256); }
-        else { v = odd ? -wthis[(size_t)k * 32 + (n - 288)] : wprev[(size_t)k * 32 + (n - 288)]; cta = 1; local = 128 + (n - 288); }
+        if (n < 256) {
+          v = lw.Wk[gi][(size_t)k * 256 + n]; cta = n >> 7; local = n & 127;
+          NL = 128; base += (size_t)16 * 2 * 32 * 32 + (size_t)step * 2 * 128 * 32;
+        } else {
+          if (n < 288) { v = odd ? wprev[(size_t)k * 32 + (n - 256)] : -wthis[(size_t)k * 32 + (n - 256)]; cta = 0; local = n - 256; }
+          else { v = odd ? -wthis[(size_t)k * 32 + (n - 288)] : wprev[(size_t)k * 32 + (n - 288)]; cta = 1; local = n - 288; }
+          NL = 32; base += (size_t)step * 2 * 32 * 32;
+        }
       } else {
         rr -= 16 * 320;
         const int step = (int)(rr / 256);

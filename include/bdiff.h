@@ -95,6 +95,12 @@ BDIFF_API int32_t bdiff_selftest_split(void* stream, int32_t variant, const floa
  * Synchronises. */
 BDIFF_API int32_t bdiff_selftest_pair(void* stream, const float* A, const float* W, float* C);
 
+/* Weight-stream layout of one layer's edge pass in tensor mode, for edge / xi hidden sizes (e_hidden, xi_hidden); no GPU
+ * needed.  out[0] = bytes packed per layer, out[1] = TMA chunks per CTA and edge tile (streamed by the producer lane,
+ * relayed by the peer CTA), out[2] = bytes of those chunks summed over both CTAs (must equal out[0]).  Returns
+ * BDIFF_EINVAL for sizes the tensor mode does not support. */
+BDIFF_API int32_t bdiff_tc_edge_stream_layout(int32_t e_hidden, int32_t xi_hidden, int64_t* out);
+
 /* Replaces: GCPNetDynamics.get_fully_connected_edge_index (gcpnet.py:1054-1066) — as an implicit plan.
  * batch_index int64[N] (sorted molecule ids, as every caller provides), mask uint8[N].  Builds the
  * per-molecule offsets the kernels enumerate edges from; *num_edges_host receives E = sum_k nact_k^2.

@@ -2,7 +2,9 @@
 """Timing of the layer megakernel k_layers_tc (BDIFF_TIMING=1), GPU only:
   * per item: for a few CTAs, the first 16 work items with their fetch time, dependency/fence wait and run time (cycles);
   * per phase: for one edge tile and one node tile per CTA, the time between consecutive stamps (one before and after
-    every accumulator wait, one after every operand publication), averaged over the CTAs."""
+    every accumulator wait, one after every operand publication), averaged over the CTAs.  An edge GCP k has two
+    accumulator waits: the U pass (gates, u_full) and the S pass + G(k)b (d_full);
+  * MMA lane: per item, cycles spent waiting for weight chunks and for operand publications, the rest issuing."""
 import os, sys
 os.environ["BDIFF_TIMING"] = "1"
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -29,12 +31,17 @@ for c in (0, 1, 50, 100, 147):
         ty = "N" if (code >> 30) & 1 else "E"
         out.append(f"{ty}{(code >> 24) & 63}.{code & 0xffffff}: fetch+{tf - t0} wait {ts - tf} run {te - ts}")
     print(f"CTA {c}:\n   " + "\n   ".join(out))
-EDGE = ["T0 assemble->publish", "wait G0", "E0 silu->publish"]
+# one label per interval between consecutive stamps: every wait has a stamp before and after it, every publication one after
+# it ("-> ..." = the short stretch from the previous publication to the next wait)
+EDGE = ["T0 assemble->publish", "E0 prefetch", "wait G0", "E0 silu->publish"]
 for k in (1, 2, 3):
-    EDGE += [f"wait G{k}a", f"E{k}a gate/vec->publish", f"wait G{k}b", f"E{k}b residual->publish"]
-EDGE += ["wait G4", "E4 gate + reduction"]
-NODE = ["T0a->publish", "T0 vectors", "wait G1a", "T0b->publish", "wait G1bc", "E1->publish", "wait G2", "E2->publish", "wait G3a",
-        "E3a->publish", "wait G3b(+G4)", "E3b->publish", "E4 PI", "wait G5", "E5 + zero"]
+    EDGE += [f"-> wait U{k}", f"wait G{k}a U pass (u_full)", f"E{k}a gate/vec->publish",
+             f"-> wait S{k}", f"wait G{k}a S pass + G{k}b", f"E{k}b residual->publish"]
+EDGE += ["m.s reduction rounds 0-3", "wait G4", "E4 gate + m.v rounds"]
+NODE = ["T0a->publish", "T0 vectors", "wait G1a", "T0b->publish"]
+for g, e in (("G1bc", "E1"), ("G2", "E2"), ("G3a", "E3a"), ("G3b(+G4)", "E3b")):
+    NODE += [f"-> wait {g}", f"wait {g}", f"{e}->publish"]
+NODE += ["E4 PI", "wait G5", "E5 + zero"]
 ph = st[256:512]
 for kind, off, names in (("edge", 0, EDGE), ("node", 32, NODE)):
     rows = ph[:148, off:off + 32]
@@ -46,8 +53,9 @@ for kind, off, names in (("edge", 0, EDGE), ("node", 32, NODE)):
     d = (rows[:, 1:nst] - rows[:, :nst - 1]).mean(0)
     tot = (rows[:, nst - 1] - rows[:, 0]).mean()
     print(f"{kind} tile: {rows.shape[0]} CTAs, {nst} stamps, total {tot:.0f} cycles")
+    assert len(names) == nst - 1, f"{kind} tile: {nst} stamps but {len(names)} phase labels"
     for i, v in enumerate(d.tolist()):
-        print(f"   {names[i] if i < len(names) else '?':32s} {v:9.0f}  {100 * v / tot:5.1f} %")
+        print(f"   {names[i]:32s} {v:9.0f}  {100 * v / tot:5.1f} %")
 
 mm = st[256 + 148:256 + 148 + 19].reshape(-1, 4)[:148 * 2]
 for kind, ty in (("edge", 0), ("node", 1)):
